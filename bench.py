@@ -190,11 +190,11 @@ class ReferenceRunner:
         assert err == 0, err
 
     def run(self, image, repeats=1):
-        """best seconds per image over `repeats` runs"""
+        """best seconds per image over `repeats` runs; the blocks of the last run are kept in self.last"""
         best = 1e30
         for _ in range(repeats):
             t0 = time.perf_counter()
-            self.lib.compress_ctx(self.ctx, image, self.cfg["block"], self.cfg["block"], threads=self.threads)
+            self.last = self.lib.compress_ctx(self.ctx, image, self.cfg["block"], self.cfg["block"], threads=self.threads)
             best = min(best, time.perf_counter() - t0)
         return best
 
@@ -228,6 +228,26 @@ def cpu_baseline(c, image, max_seconds=20.0):
                       % (reps + 1, threads, hi["affinity"], hi["cgroup_quota_cores"])}
 
 
+DUMP_LIMIT = 63 << 20     # the dump stays under 64 MiB, .npy headers included
+
+
+def dump_outputs(path, outputs):
+    """Write each payload as <path>/<name>.npy: one row of 16 float32 byte values per block. Payloads over DUMP_LIMIT in
+    all are cut to the same fixed, seeded sample of block rows, whose indices go to <name>_rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    n = sum(a.size for a in outputs.values()) // 16
+    # a row takes 64 bytes, and 8 more for its index once the rows are sampled
+    frac = 1.0 if n * 64 <= DUMP_LIMIT else DUMP_LIMIT / (n * 72)
+    for name, blocks in outputs.items():
+        rows = np.asarray(blocks, dtype=np.uint8).reshape(-1, 16)
+        if frac < 1.0:
+            keep = int(len(rows) * frac)
+            idx = np.sort(np.random.default_rng(0).choice(len(rows), size=keep, replace=False))
+            rows = rows[idx]
+            np.save(os.path.join(path, name + "_rows.npy"), idx.astype(np.float64))
+        np.save(os.path.join(path, name + ".npy"), rows.astype(np.float32))
+
+
 def traffic_from_profile():
     """DRAM bytes of one pipeline pass (all stage-kernel launches of one image), summed from the committed ncu capture."""
     try:
@@ -248,7 +268,11 @@ def main():
                     help="N > 1: which library path the e2e figure uses (auto = batch, and the slab numbers as an extra object)")
     ap.add_argument("--images-per-gpu", type=int, default=0, help="batch mode: images per rank and step (default 8: BASELINE.json configs[4] is 64 images over 8 GPUs)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the blocks the last timed step produced (N > 1: every rank's payload as gathered on rank 0) to DIR/*.npy, "
+                                                           "so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -256,7 +280,7 @@ def main():
     cfg = CONFIGS[c]
     DIM, BLOCK = cfg["dim"], cfg["block"]
     W = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 0)
-    K = max(args.steps, 1)
+    K = args.steps
     metric = "Mtexels/s at 4K RGBA 6x6 -medium" if c in (1, 4) else "Mtexels/s at %s" % workload_name(c).split(" (")[0]
     config = {"workload": workload_name(c), "block": "%dx%d" % (BLOCK, BLOCK), "preset": cfg["preset"], "profile": cfg["pname"],
               "l2": "flushed between timed steps (256 MiB memset)"}
@@ -276,6 +300,8 @@ def main():
             runner.run(image)
         dt = (time.perf_counter() - t0) / K
         runner.close()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"blocks": runner.last})
         v = DIM * DIM / dt / 1e6
         line = {"impl": "reference", "metric": metric, "value": v, "unit": "Mtexels/s", "n_gpus": args.gpus, "steps": K, "warmup": W,
                 "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -347,6 +373,13 @@ def main():
     launches = ctx.launch_count() - launches0
     dev_ms = sum(a.elapsed_time(b) for a, b in evs) / K
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # copied before the passes below overwrite d_out
+        if world > 1:
+            outputs = {"blocks_rank%d" % r: buf.cpu().numpy() for r, buf in enumerate(gather_list)}
+        else:
+            outputs = {"blocks": d_out.cpu().numpy()}
+        dump_outputs(args.dump_outputs, outputs)
 
     # kernel-only duration (roofline): events tightly around the kernel on its stream, no gather
     kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(min(K, 5))]

@@ -326,6 +326,154 @@ def ref_lib():
     return AstcencLib(REF_SO)
 
 
+# ---- the reference build's answers, recorded ---------------------------------------------------------------------
+# The tests compare with the unmodified reference build through the `reference` fixture. That build is made from the
+# reference's sources, which a checkout of this repository does not have, so the fixture answers from
+# tests/golden/golden_reference.npz: what the build returned for every call the tests make (tests/golden/make_golden_reference.py
+# records it). Each call is keyed by a hash of its method and arguments (inputs included byte for byte, the caller's thread
+# count excluded: the reference's output does not depend on it). Small outputs, and the ones a test feeds on to the next
+# step, are stored whole; the others as their SHA-256, which same_bytes() compares against.
+REF_RECORD = os.path.join(ROOT, "tests", "golden", "golden_reference.npz")
+
+
+def _feed(h, x):
+    if isinstance(x, np.ndarray):
+        h.update(b"a" + x.dtype.str.encode() + repr(x.shape).encode())
+        h.update(np.ascontiguousarray(x).tobytes())
+    elif isinstance(x, (list, tuple)):
+        h.update(b"l%d" % len(x))
+        for y in x:
+            _feed(h, y)
+    elif isinstance(x, (bool, int, float, np.integer, np.floating)):
+        h.update(b"n" + repr(float(x)).encode())
+    else:
+        h.update(b"s" + repr(x).encode())
+
+
+def call_key(method, args):
+    import hashlib
+    h = hashlib.sha256(method.encode())
+    _feed(h, list(args))
+    return h.digest()[:8]
+
+
+def output_bytes(x):
+    if isinstance(x, np.ndarray):
+        return np.ascontiguousarray(x).tobytes()
+    if isinstance(x, list):
+        return b"".join(x)
+    if isinstance(x, dict):
+        return np.array([x.get(k, np.nan) for k in METRIC_FIELDS], dtype=np.float64).tobytes()
+    return bytes(x)
+
+
+def output_digest(x):
+    import hashlib
+    return hashlib.sha256(output_bytes(x)).digest()[:16]
+
+
+class Recorded:
+    """A reference output kept as its digest only."""
+
+    def __init__(self, digest):
+        self.digest = digest
+
+
+def same_bytes(got, want):
+    """`got` has exactly the bytes of the reference's output `want` (an array, a list of block-info structs, or a Recorded digest)."""
+    if isinstance(want, Recorded):
+        return output_digest(got) == want.digest
+    return output_bytes(got) == output_bytes(want)
+
+
+class RecordedReference:
+    """Stands in for AstcencLib(REF_SO) with the calls the tests make. With `live` (an AstcencLib on the reference build)
+    every call runs the build and is recorded, and save() writes the record; without it, calls are answered from the record."""
+
+    KEEP_BYTES = 1024
+
+    def __init__(self, path=REF_RECORD, live=None):
+        self.path, self.live = path, live
+        self.kept, self.digests, self.pinned, self.last = {}, {}, set(), None
+        if live is None:
+            z = np.load(path)
+            off, blob = z["kept_off"], z["kept_blob"]
+            self.kept = {bytes(k): blob[off[i]:off[i + 1]].tobytes() for i, k in enumerate(z["kept_keys"])}
+            self.digests = {bytes(k): bytes(d) for k, d in zip(z["digest_keys"], z["digests"])}
+
+    def _call(self, method, args, run):
+        key = call_key(method, args)
+        self.last = key
+        if self.live is not None:
+            out = run(self.live)
+            self.kept[key] = output_bytes(out)
+            return out
+        if key in self.kept:
+            return self.kept[key]
+        if key in self.digests:
+            return Recorded(self.digests[key])
+        raise KeyError("%s: no recorded reference output for these arguments (tests/golden/make_golden_reference.py records them)" % method)
+
+    def pin(self):
+        """Store the last call's output whole: a test feeds it on as input."""
+        self.pinned.add(self.last)
+
+    def save(self):
+        kept = {k: v for k, v in self.kept.items() if k in self.pinned or len(v) <= self.KEEP_BYTES}
+        import hashlib
+        digests = {k: hashlib.sha256(v).digest()[:16] for k, v in self.kept.items() if k not in kept}
+        ks = sorted(kept)
+        off = np.cumsum([0] + [len(kept[k]) for k in ks]).astype(np.int64)
+        blob = np.frombuffer(b"".join(kept[k] for k in ks), dtype=np.uint8)
+        dk = sorted(digests)
+        np.savez_compressed(self.path, kept_keys=np.array([np.frombuffer(k, np.uint8) for k in ks]).reshape(-1, 8), kept_off=off, kept_blob=blob,
+                            digest_keys=np.array([np.frombuffer(k, np.uint8) for k in dk]).reshape(-1, 8),
+                            digests=np.array([np.frombuffer(digests[k], np.uint8) for k in dk]).reshape(-1, 16))
+        return len(ks), len(dk)
+
+    @staticmethod
+    def _array(raw, dtype, shape):
+        if isinstance(raw, Recorded):
+            return raw
+        return np.frombuffer(raw, dtype=dtype).reshape(shape).copy() if isinstance(raw, bytes) else raw
+
+    def compress(self, img, profile, bx, by, quality, flags=0, swz=(0, 1, 2, 3), threads=1):
+        raw = self._call("compress", (img, profile, bx, by, quality, flags, tuple(swz)),
+                         lambda L: L.compress(img, profile, bx, by, quality, flags, swz=swz, threads=threads))
+        return self._array(raw, np.uint8, (-1,))
+
+    def compress_volume(self, vol, profile, bx, by, bz, quality, flags=0, swz=(0, 1, 2, 3), threads=1):
+        raw = self._call("compress_volume", (vol, profile, bx, by, bz, quality, flags, tuple(swz)),
+                         lambda L: L.compress_volume(vol, profile, bx, by, bz, quality, flags, swz=swz, threads=threads))
+        return self._array(raw, np.uint8, (-1,))
+
+    def decompress_volume(self, blocks, w, h, d, profile, bx, by, bz, out_type=TYPE_U8, flags=0, swz=(0, 1, 2, 3), quality=PRE_MEDIUM):
+        raw = self._call("decompress_volume", (np.asarray(blocks, dtype=np.uint8), w, h, d, profile, bx, by, bz, out_type, flags, tuple(swz), quality),
+                         lambda L: L.decompress_volume(blocks, w, h, d, profile, bx, by, bz, out_type=out_type, flags=flags, swz=swz, quality=quality))
+        return self._array(raw, AstcencLib.NP_TYPES[out_type], (d, h, w, 4))
+
+    def block_infos(self, blocks, profile, bx, by, flags=0, quality=PRE_MEDIUM, bz=1):
+        raw = self._call("block_infos", (np.asarray(blocks, dtype=np.uint8), profile, bx, by, flags, quality, bz),
+                         lambda L: L.block_infos(blocks, profile, bx, by, flags=flags, quality=quality, bz=bz))
+        if isinstance(raw, bytes):
+            n = C.sizeof(BlockInfo)
+            return [raw[i:i + n] for i in range(0, len(raw), n)]
+        return raw
+
+    def config(self, profile, bx, by, quality, flags=0):
+        raw = self._call("config", (profile, bx, by, quality, flags), lambda L: L.config(profile, bx, by, quality, flags))
+        return Config.from_buffer_copy(raw) if isinstance(raw, bytes) else raw
+
+    def cli_error_metrics(self, img1, img2, hdr=False, normal=False, components=4, fstop_lo=-10, fstop_hi=10):
+        """What the reference command line tool prints for the pair (ref_error_metrics)."""
+        raw = self._call("cli_error_metrics", (img1, img2, hdr, normal, components, fstop_lo, fstop_hi),
+                         lambda L: ref_error_metrics(img1, img2, hdr=hdr, normal=normal, components=components, fstop_lo=fstop_lo, fstop_hi=fstop_hi))
+        if isinstance(raw, bytes):
+            v = np.frombuffer(raw, dtype=np.float64)
+            return {k: float(x) for k, x in zip(METRIC_FIELDS, v) if not np.isnan(x)}
+        return raw
+
+
 class OracleConfig(C.Structure):
     _fields_ = [
         ("profile", C.c_int), ("flags", C.c_uint), ("block_x", C.c_uint), ("block_y", C.c_uint), ("block_z", C.c_uint),

@@ -118,4 +118,4 @@ def test_get_block_info_matches_reference(pkg, reference, golden):
     for blocks, prof, bx, by in streams:
         want = reference.block_infos(blocks, prof, bx, by)
         got = prod.block_infos(blocks, prof, bx, by)
-        assert got == want
+        assert same_bytes(got, want)

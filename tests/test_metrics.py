@@ -48,8 +48,7 @@ def test_oracle_matches_reference_golden():
     assert n >= 12
 
 
-@pytest.mark.skipif(not have_ref_metrics(), reason="oracle/_ref/libastcenc_ref_metrics.so not built")
-def test_oracle_matches_reference_live():
+def test_oracle_matches_reference_live(reference):
     orc = Oracle()
     rng = np.random.default_rng(77)
     for trial in range(6):
@@ -57,7 +56,7 @@ def test_oracle_matches_reference_live():
         a = rng.integers(0, 256, (h, w, 4), dtype=np.uint8)
         b = np.clip(a.astype(int) + rng.integers(-20, 21, a.shape), 0, 255).astype(np.uint8)
         comps = int(rng.integers(1, 5))
-        r = ref_error_metrics(a, b, normal=True, components=comps)
+        r = reference.cli_error_metrics(a, b, normal=True, components=comps)
         o = orc.error_metrics(a, b, normal=True, components=comps)
         for k, v in r.items():
             assert abs(o[k] - v) <= PRINT_TOL[k], (trial, k, o[k], v)
